@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference ...                      (the CPU restatement of the reference on the host cores)
+    python bench.py ... --dump-outputs DIR                     (also write the last timed step's results to DIR/*.npy)
 
 One "step" = one pass of the decode hot path over one batch of synthetic frames resident in HBM:
   K1 fused preprocess+ahash+colour -> K1x exact-walk check -> bit pack -> RS(155,125) -> fountain-chunk masks,
@@ -60,7 +61,34 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-sample", type=int, default=0, help="frames per step for --impl reference (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed (rank 0) as DIR/<name>.npy: the chunk records of "
+                         "a fixed, seeded sample of frames, and every frame's chunk mask and frame flags (float32, at most 64 MB)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.camera or args.fountain):
+        ap.error("--dump-outputs applies to the decode path (not to --impl reference, --camera or --fountain)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, chunks, mask, fflags):
+    """The last step's results as float32 .npy files.  chunks is (frames, data_bytes) uint8; its rows go out for a sorted
+    sample of frames drawn with a fixed seed (all of them when they fit), so that two builds run with the same arguments
+    can be compared file by file.  mask (int32, < 2^24) and fflags (uint8) are exact in float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    B, row = chunks.shape
+    small = 4 * 3 * B + 4 * 4096                                        # chunk_mask, frame_flags, the row index; .npy headers
+    n = min(B, (DUMP_LIMIT_BYTES - small) // (4 * row))
+    rows = np.sort(np.random.default_rng(0xD0).choice(B, n, replace=False)) if n < B else np.arange(B)
+    sel = torch.from_numpy(rows).to(chunks.device)
+    arrays = {"chunks": chunks.index_select(0, sel), "chunks_rows": rows, "chunk_mask": mask, "frame_flags": fflags}
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def measured_peak_gbs():
@@ -360,6 +388,8 @@ def run_ours(args):
         wrong = int((bits & ~same).sum().item())
         parity = "%d of %d chunks decoded, %d frames complete; decoded chunks != payload: %d" % (
             good, B * cpf, int(bits.all(dim=1).sum().item()), wrong)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, chunks.view(B, info.data_bytes), mask.view(B), fflags)
 
     # ---- end to end through the host-pointer C ABI: pinned host frames -> cb200_decode_fountain -> host chunks
     e2e = None

@@ -5,6 +5,7 @@
 nvcc cross-compiles without a GPU; the built .so is git-ignored but travels to the GPU box with the repo snapshot.
 Every .cu is compiled to its own object (in parallel, only when it or a header changed) and the objects are linked."""
 import os
+import shutil
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -88,25 +89,21 @@ def build_facade(force=False, verbose=False):
 
 
 WIREHAIR_LIB = os.path.join(HERE, "lib", "libwirehair.so")
-WIREHAIR_SRC = "/root/reference/src/third_party_lib/wirehair"
+WIREHAIR_BUILT = os.path.join(HERE, "..", "oracle", "_ref", "libwirehair.so")
 
 
 def build_wirehair(force=False, verbose=False):
-    """wirehair -- the reference's third-party fountain codec (P15, stays on the rank-0 host) -- as a shared library of its own:
-    its four translation units compiled UNMODIFIED from where they lie in the reference checkout (nothing is copied into this
-    repository).  Where the checkout is absent (the GPU box) the prebuilt file that travelled with the snapshot is used.
+    """wirehair -- the reference's third-party fountain codec (P15, stays on the rank-0 host) -- next to the product's libraries.
+    Its sources are not part of this repository: `make -C oracle ref` compiles them unmodified from the reference checkout into
+    oracle/_ref/libwirehair.so, and this installs that file as lib/libwirehair.so, where the facade and FountainSink look for it.
     The product binds it at run time (cb200_sink_create_wirehair), exactly as libcimbar links it."""
-    if not os.path.isdir(WIREHAIR_SRC):
+    if not os.path.exists(WIREHAIR_BUILT):
         return WIREHAIR_LIB if os.path.exists(WIREHAIR_LIB) else None
-    srcs = [os.path.join(WIREHAIR_SRC, f) for f in ("wirehair.cpp", "gf256.cpp", "WirehairCodec.cpp", "WirehairTools.cpp")]
-    if not force and os.path.exists(WIREHAIR_LIB) and all(os.path.getmtime(x) <= os.path.getmtime(WIREHAIR_LIB) for x in srcs):
-        return WIREHAIR_LIB
-    os.makedirs(os.path.dirname(WIREHAIR_LIB), exist_ok=True)
-    cmd = ["g++", "-std=c++11", "-O3", "-mavx2", "-mssse3", "-fPIC", "-shared", "-I" + os.path.join(WIREHAIR_SRC, "include"),
-           "-I" + WIREHAIR_SRC, "-o", WIREHAIR_LIB] + srcs
-    if verbose:
-        print(" ".join(cmd))
-    subprocess.check_call(cmd)
+    if force or not os.path.exists(WIREHAIR_LIB) or os.path.getmtime(WIREHAIR_LIB) < os.path.getmtime(WIREHAIR_BUILT):
+        os.makedirs(os.path.dirname(WIREHAIR_LIB), exist_ok=True)
+        if verbose:
+            print("install %s -> %s" % (WIREHAIR_BUILT, WIREHAIR_LIB))
+        shutil.copy2(WIREHAIR_BUILT, WIREHAIR_LIB)
     return WIREHAIR_LIB
 
 

@@ -2,6 +2,7 @@
 OpenCV-free sources (oracle/_ref/libcimbar_ref.so).  TEST INFRASTRUCTURE ONLY: imported by tests/,
 __graft_entry__.smoke() and bench.py's cpu_baseline legs -- never by libcimbar_b200/."""
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -249,6 +250,22 @@ class Ref:
     def grid_args(self, m, padding=0):
         return (m.cell_spacing_x, m.cell_spacing_y, m.cells_per_col_x, m.cells_per_col_y, m.cell_offset + padding,
                 m.corner_padding_x, m.corner_padding_y)
+
+
+def digest(*parts):
+    """SHA-256 over the parts in order (arrays by their bytes, anything else by its repr): the form in which
+    tests/golden/ref_outputs.json keeps the reference's results"""
+    h = hashlib.sha256()
+    for p in parts:
+        h.update(np.ascontiguousarray(p).tobytes() if isinstance(p, np.ndarray) else repr(p).encode())
+    return h.hexdigest()
+
+
+def ref_outputs():
+    """the reference's results for the inputs of the *_is_the_references / *_matches_* tests, written by
+    tests/golden/make_ref_goldens.py from oracle/_ref (the reference's sources compiled unmodified)"""
+    with open(os.path.join(GOLDEN_DIR, "ref_outputs.json")) as f:
+        return json.load(f)
 
 
 _manifest = None

@@ -1,106 +1,150 @@
 """Checks the restatement (oracle/cimbar_oracle.c) against the reference's own OpenCV-free code compiled
 unmodified into oracle/_ref/libcimbar_ref.so (oracle/Makefile `ref`, oracle/ref_shim.cpp):
 libcorrect RS incl. its failure/miscorrection behaviour, the flood walk on the real std::priority_queue,
-cell geometry, interleave, the RS->aligned_stream->escrow stack, FountainMetadata, wirehair."""
+cell geometry, interleave, the RS->aligned_stream->escrow stack, FountainMetadata, wirehair.
+
+Each check runs one fixed input sequence through a "side" -- OracleSide here, RefSide (tests/golden/make_ref_goldens.py)
+for the reference -- and compares the digest of what came out with the reference's, stored in tests/golden/ref_outputs.json."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
-from oracle_lib import Oracle, Ref, _ptr
+from oracle_lib import Oracle, _ptr, digest, ref_outputs
 
 ORA = Oracle()
-try:
-    REF = Ref()
-except (FileNotFoundError, OSError) as e:  # pragma: no cover
-    REF = None
-    pytestmark = pytest.mark.skip(reason=f"oracle/_ref not available: {e}")
 
 MODES = [68, 4, 8, 67, 66]
+INTERLEAVE_ARGS = [(12400, 155, 2), (12400, 155, 1), (12400, 0, 2), (8592, 179, 2), (5376, 168, 2)]
+WALK_MODES, WALK_NOISE = [68, 67, 66], [0, 3, 30, 100]
+RS_CODES = [(30, 155), (33, 168), (36, 179), (40, 216), (15, 155)]
+STREAM_MODES = [68, 4, 67, 66]
 
 
-@pytest.mark.parametrize("mode", MODES)
-def test_cell_positions_and_adjacency(mode):
+class OracleSide:
+    """the restatement, behind the calls the reference side makes"""
+
+    def cell_positions(self, m, xs, ys):
+        return ORA.lib.cbo_cell_positions(C.byref(m), 0, _ptr(xs, C.c_int), _ptr(ys, C.c_int))
+
+    def adjacent(self, m, xs, idx, out):
+        ORA.lib.cbo_adjacent(C.byref(m), _ptr(xs, C.c_int), m.total_cells, idx, _ptr(out, C.c_int))
+
+    def interleave_reverse(self, args, out):
+        ORA.lib.cbo_interleave_reverse(*args, _ptr(out, C.c_uint))
+
+    def flood_walk(self, m, seed, noise, o, d, c):
+        return ORA.lib.cbo_flood_walk_synthetic(C.byref(m), seed, noise, _ptr(o, C.c_uint16), _ptr(d, C.c_int8), _ptr(c))
+
+    def fuzzy_ahash(self, bits, w, wx, wy, all_, out):
+        ORA.lib.cbo_fuzzy_ahash(_ptr(bits), w, wx, wy, all_, out)
+
+    def rs_create(self, parity):
+        return ORA.lib.cbo_rs_create(parity)
+
+    def rs_destroy(self, h):
+        ORA.lib.cbo_rs_destroy(h)
+
+    def rs_encode(self, h, msg, out):
+        return ORA.lib.cbo_rs_encode(h, _ptr(msg), msg.size, _ptr(out))
+
+    def rs_decoder(self, encoder, parity):
+        return encoder          # the restatement decodes with the object that encoded the blocks
+
+    def rs_decode(self, h, blk, out):
+        return ORA.lib.cbo_rs_decode(h, _ptr(blk), blk.size, _ptr(out))
+
+    def rs_stream(self, parity, block, raw, sym_len):
+        """Decoder::decode: the corrected bytes of the symbol stream"""
+        return ORA.rs_stream(parity, block, raw[:sym_len])[0]
+
+    def rs_align(self, m, raw, sym_len, col_len):
+        """Decoder::decode_fountain: (bytes written, chunks written, the chunks) -- rs_stream + align_chunks"""
+        parity, block = m.ecc_bytes, m.ecc_block_size
+        msg, nblocks = block - parity, ORA.capacity(m) // block
+        data = np.zeros(nblocks * msg, np.uint8)
+        okall = np.zeros(nblocks, np.uint8)
+        o1, k1 = ORA.rs_stream(parity, block, raw[:sym_len])
+        data[:o1.size], okall[:k1.size] = o1, k1
+        if col_len:
+            o2, k2 = ORA.rs_stream(parity, block, raw[sym_len:])
+            data[o1.size:], okall[k1.size:] = o2, k2
+        chunks = np.zeros((m.chunks_per_frame, m.chunk_size), np.uint8)
+        mask = C.c_uint32(0)
+        good = ORA.lib.cbo_align_chunks(_ptr(data), _ptr(okall), nblocks, msg, m.chunk_size, _ptr(chunks), C.byref(mask))
+        used = bin(mask.value).count("1")
+        assert good == used * m.chunk_size
+        return good, used, chunks
+
+    def md_pack(self, eid, size, bid, out):
+        ORA.lib.cbo_md_pack(eid, size, bid, _ptr(out))
+
+    def md_fields(self, a):
+        return ORA.lib.cbo_md_file_size(_ptr(a)), ORA.lib.cbo_md_block_id(_ptr(a)), ORA.lib.cbo_md_encode_id(_ptr(a))
+
+
+def cell_positions_and_adjacency(side, mode):
     m = ORA.mode(mode)
     n = m.total_cells
     xs, ys = np.zeros(n, np.int32), np.zeros(n, np.int32)
-    rxs, rys = np.zeros(n, np.int32), np.zeros(n, np.int32)
-    assert ORA.lib.cbo_cell_positions(C.byref(m), 0, _ptr(xs, C.c_int), _ptr(ys, C.c_int)) == n
-    assert REF.lib.ref_cell_positions(*REF.grid_args(m), _ptr(rxs, C.c_int), _ptr(rys, C.c_int)) == n
-    assert np.array_equal(xs, rxs) and np.array_equal(ys, rys)
-    if mode == 68:  # CellPositionsTest.cpp:11-27
-        assert (xs[0], ys[0]) == (62, 8) and n == 12400
-    a, ra = np.zeros(4, np.int32), np.zeros(4, np.int32)
+    assert side.cell_positions(m, xs, ys) == n
+    out = [xs, ys]
     rng = np.random.default_rng(1)
     for idx in list(rng.integers(0, n, 300)) + [0, n - 1, 99, 100, 599, 600, 711, 712, n - 600, n - 601]:
-        ORA.lib.cbo_adjacent(C.byref(m), _ptr(xs, C.c_int), n, int(idx), _ptr(a, C.c_int))
-        REF.lib.ref_adjacent(*REF.grid_args(m), int(idx), _ptr(ra, C.c_int))
-        assert np.array_equal(a, ra), idx
+        a = np.zeros(4, np.int32)
+        side.adjacent(m, xs, int(idx), a)
+        out.append(a)
+    return out
 
 
-@pytest.mark.parametrize("args", [(12400, 155, 2), (12400, 155, 1), (12400, 0, 2), (8592, 179, 2), (5376, 168, 2)])
-def test_interleave_reverse(args):
-    size = args[0]
-    a, b = np.zeros(size, np.uint32), np.zeros(size, np.uint32)
-    ORA.lib.cbo_interleave_reverse(*args, _ptr(a, C.c_uint))
-    REF.lib.ref_interleave_reverse(*args, _ptr(b, C.c_uint))
-    assert np.array_equal(a, b)
-    if args == (12400, 155, 1):  # InterleaveTest.cpp:14-58
-        assert a[1] == 80
+def interleave_reverse(side, args):
+    a = np.zeros(args[0], np.uint32)
+    side.interleave_reverse(args, a)
+    return a
 
 
-@pytest.mark.parametrize("mode", [68, 67, 66])
-@pytest.mark.parametrize("noise", [0, 3, 30, 100])
-def test_flood_walk_matches_std_priority_queue(mode, noise):
+def flood_walks(side, mode, noise):
     m = ORA.mode(mode)
     n = m.total_cells
+    out = []
     for seed in range(4):
         o, d, c = np.zeros(n, np.uint16), np.zeros(2 * n, np.int8), np.zeros(n, np.uint8)
-        ro, rd, rc = np.zeros(n, np.uint16), np.zeros(2 * n, np.int8), np.zeros(n, np.uint8)
-        assert ORA.lib.cbo_flood_walk_synthetic(C.byref(m), seed, noise, _ptr(o, C.c_uint16), _ptr(d, C.c_int8), _ptr(c)) == n
-        assert REF.lib.ref_flood_walk_synthetic(*REF.grid_args(m), seed, noise, _ptr(ro, C.c_uint16), _ptr(rd, C.c_int8), _ptr(rc)) == n
-        assert np.array_equal(o, ro) and np.array_equal(d, rd) and np.array_equal(c, rc)
-        assert sorted(o.tolist()) == list(range(n))
-    if mode == 68 and noise == 0:  # FloodDecodePositionsTest.cpp:11-129 seeds; SURVEY appendix A.6 clean walk order
-        assert o[:4].tolist() == [0, 12399, 99, 12300]
+        assert side.flood_walk(m, seed, noise, o, d, c) == n
+        out += [o, d, c]
+    return out
 
 
-def test_fuzzy_ahash_vs_reference_extractors():
+def fuzzy_ahashes(side):
     rng = np.random.default_rng(7)
     w, h = 64, 40
     bits = rng.integers(0, 256, w * h // 8, dtype=np.uint8)
-    mine, ref = (C.c_uint64 * 9)(), (C.c_uint64 * 9)()
+    out = []
     for _ in range(200):
         wx, wy, all_ = int(rng.integers(0, w - 10)), int(rng.integers(0, h - 10)), int(rng.integers(0, 2))
-        ORA.lib.cbo_fuzzy_ahash(_ptr(bits), w, wx, wy, all_, mine)
-        REF.lib.ref_fuzzy_ahash(_ptr(bits), bits.size, w, wx, wy, all_, ref)
-        assert list(mine) == list(ref)
+        r = (C.c_uint64 * 9)()
+        side.fuzzy_ahash(bits, w, wx, wy, all_, r)
+        out.append(list(r))
+    return out
 
 
-def _rs_pair(parity):
-    o = ORA.lib.cbo_rs_create(parity)
-    r = REF.lib.ref_rs_create(parity)
-    return o, r
-
-
-def test_rs_known_answer():
+def rs_known_answer(side):
     # reed_solomon_streamTest.cpp:23: RS(155,140) parity of the ASCII digits message
     msg = np.frombuffer((b"0123456789" * 14), dtype=np.uint8).copy()
-    o, r = _rs_pair(15)
-    enc, renc = np.zeros(255, np.uint8), np.zeros(255, np.uint8)
-    assert ORA.lib.cbo_rs_encode(o, _ptr(msg), 140, _ptr(enc)) == 255
-    assert REF.lib.ref_rs_encode2(r, _ptr(msg), 140, _ptr(renc)) == 255
-    assert np.array_equal(enc[:155], renc[:155])
-    assert enc[140:155].tobytes().hex() == "a4740203 72c3adf2 60c5b69e 267873".replace(" ", "")
+    h = side.rs_create(15)
+    enc = np.zeros(255, np.uint8)
+    assert side.rs_encode(h, msg, enc) == 255
+    side.rs_destroy(h)
+    return enc[:155]
 
 
-@pytest.mark.parametrize("parity,block", [(30, 155), (33, 168), (36, 179), (40, 216), (15, 155)])
-def test_rs_decode_matches_libcorrect_including_failures(parity, block):
+def rs_decode_trials(side, parity, block):
+    """1500 blocks with 0 .. parity + 8 symbol errors (and some pure noise), encoded by the restatement, decoded by `side` with
+    one persistent decoder object (libcorrect keeps state across calls): [(trial, errors, message, returned, decoded)]"""
     rng = np.random.default_rng(parity * 1000 + block)
-    o, r = _rs_pair(parity)
+    o = ORA.lib.cbo_rs_create(parity)
+    h = side.rs_decoder(o, parity)
     msg_len = block - parity
-    n_fail = n_miscorrect = 0
-    # one persistent decoder object per side: libcorrect keeps state across calls
+    trials = []
     for trial in range(1500):
         msg = rng.integers(0, 256, msg_len, dtype=np.uint8)
         enc = np.zeros(255, np.uint8)
@@ -114,25 +158,21 @@ def test_rs_decode_matches_libcorrect_including_failures(parity, block):
         blk[pos] ^= rng.integers(1, 256, nerr, dtype=np.uint8)
         if trial % 97 == 0:
             blk = rng.integers(0, 256, block, dtype=np.uint8)  # pure noise
-        a, b = np.zeros(256, np.uint8), np.zeros(256, np.uint8)
-        na = ORA.lib.cbo_rs_decode(o, _ptr(blk), block, _ptr(a))
-        nb = REF.lib.ref_rs_decode2(r, _ptr(blk), block, _ptr(b))
-        assert na == nb, (trial, nerr)
-        if nb > 0:
-            assert np.array_equal(a[:msg_len], b[:msg_len]), (trial, nerr)
-            if nerr <= t:
-                assert np.array_equal(a[:msg_len], msg)
-            elif not np.array_equal(b[:msg_len], msg):
-                n_miscorrect += 1
-        else:
-            n_fail += 1
-    assert n_fail > 0  # the sweep really exercised libcorrect's failure path
+        a = np.zeros(256, np.uint8)
+        n = side.rs_decode(h, blk, a)
+        trials.append((trial, nerr, msg, n, a[:msg_len].copy()))
+    if h != o:
+        side.rs_destroy(h)
     ORA.lib.cbo_rs_destroy(o)
-    REF.lib.ref_rs_destroy(r)
+    return trials
 
 
-@pytest.mark.parametrize("mode", [68, 4, 67, 66])
-def test_rs_stream_and_aligned_chunks_match_reference_stack(mode):
+def rs_decode_outputs(trials):
+    """what the comparison covers: the return value of every decode, and the message wherever one came back"""
+    return [np.array([n for _, _, _, n, _ in trials], np.int64)] + [a for _, _, _, n, a in trials if n > 0]
+
+
+def rs_stream_and_aligned_chunks(side, mode):
     m = ORA.mode(mode)
     rng = np.random.default_rng(mode)
     cap = ORA.capacity(m)
@@ -144,6 +184,7 @@ def test_rs_stream_and_aligned_chunks_match_reference_stack(mode):
     else:
         sym_len, col_len = ORA.capacity(m, m.symbol_bits), ORA.capacity(m, m.color_bits)
     rs = ORA.lib.cbo_rs_create(parity)
+    out = []
     for trial in range(40):
         payload = rng.integers(0, 256, nblocks * msg, dtype=np.uint8)
         raw = np.zeros(cap, np.uint8)
@@ -162,48 +203,96 @@ def test_rs_stream_and_aligned_chunks_match_reference_stack(mode):
             bad.add(nblocks - 1)
         for b in bad:
             raw[b * block:b * block + parity] = rng.integers(0, 256, parity, dtype=np.uint8)
-        # (a) Decoder::decode semantics
-        out, ok = ORA.rs_stream(parity, block, raw[:sym_len])
-        ref_out = np.zeros(nblocks * msg + 16, np.uint8)
-        n = REF.lib.ref_rs_stream(parity, block, _ptr(raw), sym_len, _ptr(ref_out))
-        assert n == out.size and np.array_equal(out, ref_out[:n])
-        # (b) Decoder::decode_fountain semantics: oracle = rs_stream + align_chunks; reference = its stream stack
-        data = np.zeros(nblocks * msg, np.uint8)
-        okall = np.zeros(nblocks, np.uint8)
-        o1, k1 = ORA.rs_stream(parity, block, raw[:sym_len])
-        data[:o1.size], okall[:k1.size] = o1, k1
-        if col_len:
-            o2, k2 = ORA.rs_stream(parity, block, raw[sym_len:])
-            data[o1.size:], okall[k1.size:] = o2, k2
-        chunks = np.zeros((m.chunks_per_frame, m.chunk_size), np.uint8)
-        mask = C.c_uint32(0)
-        good = ORA.lib.cbo_align_chunks(_ptr(data), _ptr(okall), nblocks, msg, m.chunk_size, _ptr(chunks), C.byref(mask))
-        rchunks = np.zeros((m.chunks_per_frame, m.chunk_size), np.uint8)
-        used = C.c_uint(0)
-        rgood = REF.lib.ref_rs_align_escrow(parity, block, _ptr(raw), sym_len, col_len, m.chunk_size, m.chunks_per_frame, _ptr(rchunks), C.byref(used))
-        assert good == rgood
-        assert used.value == bin(mask.value).count("1") and good == used.value * m.chunk_size
-        assert np.array_equal(chunks, rchunks)
+        # (a) Decoder::decode semantics; (b) Decoder::decode_fountain semantics
+        stream = side.rs_stream(parity, block, raw, sym_len)
+        good, used, chunks = side.rs_align(m, raw, sym_len, col_len)
+        out += [stream.size, stream, good, used, chunks]
     ORA.lib.cbo_rs_destroy(rs)
+    return out
+
+
+def fountain_metadata(side):
+    rng = np.random.default_rng(3)
+    out = []
+    for _ in range(200):
+        eid, size, bid = int(rng.integers(0, 256)), int(rng.integers(0, 1 << 25)), int(rng.integers(0, 65536))
+        a = np.zeros(6, np.uint8)
+        side.md_pack(eid, size, bid, a)
+        fields = side.md_fields(a)
+        assert fields == (size, bid, eid & 0x7F)
+        out += [a, fields]
+    return out
+
+
+@pytest.mark.parametrize("mode", MODES)
+def test_cell_positions_and_adjacency(mode):
+    out = cell_positions_and_adjacency(OracleSide(), mode)
+    if mode == 68:  # CellPositionsTest.cpp:11-27
+        assert (out[0][0], out[1][0]) == (62, 8) and out[0].size == 12400
+    assert digest(*out) == ref_outputs()["cell_positions_and_adjacency"][str(mode)]
+
+
+@pytest.mark.parametrize("args", INTERLEAVE_ARGS)
+def test_interleave_reverse(args):
+    a = interleave_reverse(OracleSide(), args)
+    if args == (12400, 155, 1):  # InterleaveTest.cpp:14-58
+        assert a[1] == 80
+    assert digest(a) == ref_outputs()["interleave_reverse"][repr(args)]
+
+
+@pytest.mark.parametrize("mode", WALK_MODES)
+@pytest.mark.parametrize("noise", WALK_NOISE)
+def test_flood_walk_matches_std_priority_queue(mode, noise):
+    out = flood_walks(OracleSide(), mode, noise)
+    n = ORA.mode(mode).total_cells
+    for o in out[0::3]:
+        assert sorted(o.tolist()) == list(range(n))
+    if mode == 68 and noise == 0:  # FloodDecodePositionsTest.cpp:11-129 seeds; SURVEY appendix A.6 clean walk order
+        assert out[0][:4].tolist() == [0, 12399, 99, 12300]
+    assert digest(*out) == ref_outputs()["flood_walk"]["%d/%d" % (mode, noise)]
+
+
+def test_fuzzy_ahash_vs_reference_extractors():
+    assert digest(fuzzy_ahashes(OracleSide())) == ref_outputs()["fuzzy_ahash"]
+
+
+def test_rs_known_answer():
+    enc = rs_known_answer(OracleSide())
+    assert enc[140:155].tobytes().hex() == "a4740203 72c3adf2 60c5b69e 267873".replace(" ", "")
+    assert digest(enc) == ref_outputs()["rs_known_answer"]
+
+
+@pytest.mark.parametrize("parity,block", RS_CODES)
+def test_rs_decode_matches_libcorrect_including_failures(parity, block):
+    trials = rs_decode_trials(OracleSide(), parity, block)
+    n_fail = 0
+    for trial, nerr, msg, n, a in trials:
+        if n > 0:
+            if nerr <= parity // 2:
+                assert np.array_equal(a, msg), (trial, nerr)
+        else:
+            n_fail += 1
+    assert n_fail > 0  # the sweep really exercised libcorrect's failure path
+    assert digest(*rs_decode_outputs(trials)) == ref_outputs()["rs_decode"]["%d/%d" % (parity, block)]
+
+
+@pytest.mark.parametrize("mode", STREAM_MODES)
+def test_rs_stream_and_aligned_chunks_match_reference_stack(mode):
+    assert digest(*rs_stream_and_aligned_chunks(OracleSide(), mode)) == ref_outputs()["rs_stream_and_aligned_chunks"][str(mode)]
 
 
 def test_fountain_metadata():
-    rng = np.random.default_rng(3)
-    a, b = np.zeros(6, np.uint8), np.zeros(6, np.uint8)
-    for _ in range(200):
-        eid, size, bid = int(rng.integers(0, 256)), int(rng.integers(0, 1 << 25)), int(rng.integers(0, 65536))
-        ORA.lib.cbo_md_pack(eid, size, bid, _ptr(a))
-        REF.lib.ref_md_pack(eid, size, bid, _ptr(b))
-        assert np.array_equal(a, b)
-        assert ORA.lib.cbo_md_file_size(_ptr(a)) == REF.lib.ref_md_file_size(_ptr(a)) == size
-        assert ORA.lib.cbo_md_block_id(_ptr(a)) == REF.lib.ref_md_block_id(_ptr(a)) == bid
-        assert ORA.lib.cbo_md_encode_id(_ptr(a)) == REF.lib.ref_md_encode_id(_ptr(a)) == eid & 0x7F
+    assert digest(*fountain_metadata(OracleSide())) == ref_outputs()["fountain_metadata"]
 
 
 def test_sample_stream_reassembles_with_reference_wirehair():
     # samples/b/tr_0..3.png are a complete 4-frame fountain stream (.github/workflows/wasm.yml:48-49):
     # oracle decode_fountain -> chunk headers -> the reference's wirehair -> recovered (zstd) file
-    from oracle_lib import load_sample
+    from oracle_lib import Ref, load_sample
+    try:
+        REF = Ref()
+    except (FileNotFoundError, OSError) as e:  # pragma: no cover
+        pytest.skip(f"oracle/_ref not available: {e}")
     m = ORA.mode(68)
     codec, size = None, None
     seen = set()
